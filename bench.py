@@ -11,7 +11,7 @@ Workloads (SURVEY.md §8d):
        128x128 texture -> RGBA MSE + 5e-4 * loss_flat (+ mIoU).
 Synthetic, seeded inputs (no dataset exists offline).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload cfg2|cfg3]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload cfg2|cfg3] [--dump-outputs DIR]
 N>1 is launched by torchrun (one rank per GPU, NCCL); every rank owns its own shard of the global batch (weak scaling).
 cfg3's collectives: SyncBN statistics of the generator and the gradient all-reduce of G / D (captured in the step's CUDA
 graph).  `--impl reference` times the reference's algorithm on the host cores (oracle/, torch CPU) on the same config.
@@ -148,22 +148,26 @@ class CudaWorkload:
     def step(self, batches):
         """One step over `batches` (one input dict per training iteration).  cfg2: render+loss fwd+bwd.  cfg3: three
         iterations (G, D, D — the reference's 1 : d_steps_per_g alternation, main.py:691), each on its own batch =
-        render+loss fwd+bwd + one GAN step with its optimiser.  cfg4: one run_reconstruction.py iteration.  cfg5: G, D, D."""
+        render+loss fwd+bwd + one GAN step with its optimiser.  cfg4: one run_reconstruction.py iteration.  cfg5: G, D, D.
+        Returns the loss and, when the step renders, each iteration's input gradients (render_step)."""
         if self.kind == "render":
-            return self.render_step(batches[0])
+            loss, grads = self.render_step(batches[0])
+            return loss, [grads]
         if self.kind == "recon":
             d = batches[0]
             return self.recon.step(d["x_real"], d["pscale"], d["ptrans"], d["rot"], d["idx"])[0], None
-        loss = None
+        loss, grads = None, []
         for it, d in enumerate(batches):
             if it == 0:
                 gl = self.gan.g_step(d["X_alpha"], d["C"])
             else:
                 gl = self.gan.d_step(d["X_tex"], d["X_alpha"], d["X_mesh"], d["C"])
             if "render" in self.kind:
-                gl = gl + self.render_step(d)[0]
+                rl, rg = self.render_step(d)
+                gl = gl + rl
+                grads.append(rg)
             loss = gl if loss is None else loss + gl
-        return loss, None
+        return loss, grads or None
 
     def render_step(self, d):
         from b3d.mesh import rgba_mse_iou
@@ -291,6 +295,29 @@ def algorithmic_bytes(B, F_=960):
             "b3d_mesh_render_fwd": B * mesh_fwd, "b3d_mesh_render_bwd": B * mesh_bwd}
 
 
+DUMP_LIMIT = 64 << 20          # bytes written in all
+
+
+def dump_outputs(out_dir, loss, grads):
+    """What the timed step returned last (CudaWorkload.step), as <out_dir>/<name>.npy in float32: the loss and, per
+    training iteration that renders, the gradients of the loss with respect to the rendered inputs.  The trained networks'
+    state is not written: Adam with betas (0, 0.9) moves every weight by about lr * sign(gradient) in its first steps, so
+    gradients at rounding level (float atomics) make that state differ from run to run of the same build."""
+    import numpy as np
+    arrays = {"loss": loss.detach().reshape(-1)}
+    for it, g in enumerate(grads or []):
+        for name, t in zip(("points", "quat", "scale", "mesh_map", "tex"), g):
+            arrays[f"iter{it}_grad_{name}"] = t
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+    stage(f"dumped {len(arrays)} arrays ({total} bytes) to {out_dir}")
+
+
 def run_cuda(args):
     import b3d
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -389,11 +416,15 @@ def run_cuda(args):
         with torch.cuda.graph(graph, capture_error_mode="thread_local" if world > 1 else "global"):
             g_loss, g_grads = wl.step(fresh(resident))
 
+    last = {}                                                # outputs of the latest step (the graph's are static)
+
     def step_resident():
         if graph is not None:
             graph.replay()
+            last["loss"], last["grads"] = g_loss, g_grads
             return g_loss
-        return wl.step(fresh(resident))[0]
+        last["loss"], last["grads"] = wl.step(fresh(resident))
+        return last["loss"]
 
     # End-to-end input pipeline (what a training loop with a prefetching loader does): the pinned host batches of step k+1
     # are uploaded into device STAGING buffers on a copy stream while step k computes; at the start of a step the staged
@@ -443,6 +474,8 @@ def run_cuda(args):
     stage("timing (resident inputs)")
     total_ms = timed(step_resident, args.steps, args.warmup)
     hi = clocks.mark() if clocks else 0
+    if args.dump_outputs and rank == 0:                      # before the later passes overwrite the graph's outputs
+        dump_outputs(args.dump_outputs, last["loss"], last["grads"])
     launches = (b3d.launch_count() - n0) // (args.steps + args.warmup)
     if graph is not None:                                    # replays do not pass through the C ABI counter
         n1 = b3d.launch_count()
@@ -771,7 +804,11 @@ def main():
     ap.add_argument("--impl", default="b3d", choices=["b3d", "reference"])
     ap.add_argument("--workload", default="cfg3", choices=sorted(WORKLOADS))
     ap.add_argument("--no-graph", action="store_true", help="launch the step eagerly instead of replaying a CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed to "
+                    "DIR/<name>.npy (float32, seeded inputs: compare two builds output for output)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and args.impl == "b3d":
         args.warmup = 3
     (run_reference if args.impl == "reference" else run_cuda)(args)

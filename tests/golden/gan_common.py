@@ -22,6 +22,32 @@ def build(gan_module, args, seed=123):
     return G, D
 
 
+def checkpoint_standin(gan_module, seed=2024):
+    """A generator_running_avg state dict in the layout of the shipped CUB checkpoint (512^2, nd = 3), built from seeds so
+    that it can travel with the tests: same-seed weights, non-trivial batch-norm running statistics, and spectral-norm
+    vectors u, v from 30 float64 power iterations (eval mode divides each weight by u^T W v with the stored vectors, as it
+    does with a trained checkpoint)."""
+    G, _ = build(gan_module, make_args(512, 3), seed=seed)
+    sd = G.state_dict()
+    g = torch.Generator().manual_seed(seed + 2)
+    with torch.no_grad():
+        for k, v in sd.items():
+            if k.endswith("running_mean"):
+                v.copy_(0.1 * torch.randn(v.shape, generator=g))
+            elif k.endswith("running_var"):
+                v.copy_(0.5 + torch.rand(v.shape, generator=g))
+        for k in [k for k in sd if k.endswith("_orig")]:
+            base = k[: -len("orig")]
+            W = sd[k].double().reshape(sd[k].shape[0], -1)
+            u = sd[base + "u"].double()
+            for _ in range(30):
+                v = torch.nn.functional.normalize(W.t() @ u, dim=0)
+                u = torch.nn.functional.normalize(W @ v, dim=0)
+            sd[base + "u"].copy_(u)
+            sd[base + "v"].copy_(v)
+    return sd
+
+
 def inputs(args, B=2, seed=5):
     g = torch.Generator().manual_seed(seed)
     R = args.texture_resolution

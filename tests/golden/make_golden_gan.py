@@ -60,13 +60,12 @@ def make(fname, res, nd, B, probe):
 
 
 def checkpoint_kat():
-    """Known-answer test from the SHIPPED checkpoint (SURVEY §8c(1)): the reference Generator, eval mode, running-average
-    weights of gan_weights/pretrained_weights_cub/checkpoint_latest.pth -> probes.  The 52 MB checkpoint is not
-    committed; __graft_entry__.build() stages a copy under tests/golden/_ckpt/ (git-ignored) when /root/reference exists."""
-    ck = "/root/reference/code/gan_weights/pretrained_weights_cub/checkpoint_latest.pth"
+    """Known-answer test of a checkpoint load (SURVEY §8c(1)): the reference Generator, eval mode, loading strictly
+    gan_common.checkpoint_standin (the shipped CUB checkpoint's layout, seeded values; the 52 MB checkpoint itself cannot
+    travel with the tests) -> probes."""
     args = GC.make_args(512, 3)
     G = ref_gan.Generator(args, 64, symmetric=True, mesh_head=True)
-    G.load_state_dict(torch.load(ck, map_location="cpu")["generator_running_avg"], strict=True)
+    G.load_state_dict(GC.checkpoint_standin(ref_gan), strict=True)
     G.eval()
     torch.manual_seed(1234)
     z, c = torch.randn(2, 64), torch.tensor([[3], [77]])

@@ -29,6 +29,13 @@ def build_net(seed=8):
     return TinyNet()
 
 
+def record(make_record, seed=0, R=32):
+    """One pseudo-GT record at texture resolution R from seeded inputs (make_record: data/pseudo_gt.py's)."""
+    g = torch.Generator().manual_seed(seed)
+    return make_record(torch.randn(3, 32, 32, generator=g) * 0.05, torch.rand(3, R, R, generator=g) * 2 - 1,
+                       (torch.rand(1, R, R, generator=g) > 0.3).float(), torch.rand(4, 16, 16, generator=g) * 2 - 1)
+
+
 def batches(n=2, B=2):
     g = torch.Generator().manual_seed(19)
     out = []

@@ -7,4 +7,7 @@ for s in pointcloud silhouette_losses mesh template renderer pose recon recon_st
   echo "== make_golden_$s.py"
   python tests/golden/make_golden_$s.py
 done
+echo "== make_golden_reference_state.py"
+python tests/golden/make_golden_reference_state.py "${REFERENCE_CODE:?set REFERENCE_CODE to the original project's code directory}"
+cp "$REFERENCE_CODE"/mesh_templates/uvsphere_{16,31}rings.obj tests/golden/
 git status --short tests/golden

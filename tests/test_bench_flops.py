@@ -1,75 +1,21 @@
-"""The FLOP numerators of bench.py's tensor-core roofline are constants taken from SURVEY App. D.  This test measures them
-again on the REFERENCE's own modules (forward hooks on every nn.Conv2d, one image, CPU) and checks the expressions bench.py
-evaluates: dense-conv FLOPs = 2 x MACs of the forward pass; per step what is actually executed (bench.py comments).
-Authoring container only (needs /root/reference)."""
+"""The FLOP numerators of bench.py's tensor-core roofline are constants taken from SURVEY App. D.  This test checks them
+against the numbers measured on the REFERENCE's own modules (forward hooks on every nn.Conv2d, one image, CPU; stored in
+tests/golden/bench_flops_reference.npz by make_golden_reference_state.py) and checks the expressions bench.py evaluates:
+dense-conv FLOPs = 2 x MACs of the forward pass; per step what is actually executed (bench.py comments)."""
 import os
 import re
-import sys
 
-import pytest
-import torch
-import torch.nn as nn
+import numpy as np
 
 from conftest import GOLDEN, ROOT
 
-REF = "/root/reference/code"
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout not present (GPU box)")
 
-
-def conv_gflops(module, run):
-    tot, hooks = {}, []
-    for name, m in module.named_modules():
-        if isinstance(m, nn.Conv2d):
-            def hook(mod, inp, out, name=name):
-                kh, kw = mod.kernel_size
-                tot[name] = tot.get(name, 0.0) + 2.0 * out.numel() * mod.in_channels * kh * kw / 1e9
-            hooks.append(m.register_forward_hook(hook))
-    with torch.no_grad():
-        run()
-    for h in hooks:
-        h.remove()
-    return tot
-
-
-@pytest.fixture(scope="module")
-def reference_modules():
-    from conftest import PKG
-    saved = {k: sys.modules.pop(k) for k in list(sys.modules) if k.split('.')[0] in ("models", "rendering", "utils", "sync_batchnorm")}
-    sys.path.remove(PKG)
-    sys.path.insert(0, REF)
-    sys.path.insert(0, GOLDEN)
-    try:
-        import gan_common as GC
-        import recon_common as RC
-        from models import gan as ref_gan
-        from models import reconstruction as ref_recon
-        out = {}
-        for res, nd in ((256, 2), (512, 3)):
-            args = GC.make_args(res, nd)
-            G, D = GC.build(ref_gan, args)
-            G.eval(); D.eval()
-            z, c, alpha, tex, mesh = GC.inputs(args, B=1)
-            g = conv_gflops(G, lambda: G(z, c))
-            d = conv_gflops(D, lambda: D(torch.cat((tex * alpha, alpha), 1), mesh, c))
-            first = sum(v for k, v in d.items() if re.fullmatch(r"d\d\.conv1", k))
-            out[res] = (sum(g.values()), sum(d.values()), first)
-        net = RC.build(ref_recon, texture_res=128).eval()
-        r = conv_gflops(net, lambda: net(torch.rand(1, 4, 256, 256)))
-        out["recon"] = (sum(r.values()), r["conv1e"])
-        return out
-    finally:
-        sys.path.remove(REF)
-        sys.path.insert(0, PKG)
-        for k in [k for k in sys.modules if k.split('.')[0] in ("models", "rendering", "utils", "sync_batchnorm")]:
-            del sys.modules[k]
-        sys.modules.update(saved)
-
-
-def test_bench_flop_constants_match_the_reference_modules(reference_modules):
+def test_bench_flop_constants_match_the_reference_modules():
     src = open(os.path.join(ROOT, "bench.py")).read()
-    g256, d256, f256 = reference_modules[256]
-    g512, d512, f512 = reference_modules[512]
-    rec, rec_first = reference_modules["recon"]
+    r = {k: float(v) for k, v in np.load(os.path.join(GOLDEN, "bench_flops_reference.npz")).items()}
+    g256, d256, f256 = r["g256"], r["d256"], r["d_first256"]
+    g512, d512, f512 = r["g512"], r["d512"], r["d_first512"]
+    rec, rec_first = r["recon"], r["recon_first"]
     # cfg3: G step 3G + 2D, two D steps G + 6D each, minus the unexecuted first-layer input gradients of the 2B batch
     m = re.search(r"gf_img = (\(3 \* 17\.09 .*\))\n", src)
     assert m, "cfg3 FLOP expression not found in bench.py"

@@ -73,18 +73,16 @@ def test_gan_steps_match_reference_golden(fname):
         assert abs(got - ref) <= 6e-2 * ref + floor, (str(name), got, ref)
 
 
-CKPT = os.path.join(GOLDEN, "_ckpt", "checkpoint_latest.pth")
-
-
-@pytest.mark.skipif(not os.path.exists(CKPT), reason="shipped checkpoint not staged (tests/golden/_ckpt, see __graft_entry__.build)")
 def test_shipped_checkpoint_known_answer():
-    """SURVEY §8c(1): the shipped generator_running_avg weights load strict into the CUDA Generator and its eval-mode
-    forward reproduces the probes the REFERENCE Generator computed from the same checkpoint on the CPU
-    (tests/golden/make_golden_gan.py:checkpoint_kat).  Eval mode: no batch statistics, no power iteration."""
+    """SURVEY §8c(1): a generator_running_avg state dict in the shipped checkpoint's layout (gan_common.checkpoint_standin:
+    seeded values, since the 52 MB checkpoint cannot travel; its layout is checked against the shipped one by
+    test_gan_hostlogic.py) loads strict into the CUDA Generator and its eval-mode forward reproduces the probes the REFERENCE
+    Generator computed from the same state dict on the CPU (tests/golden/make_golden_gan.py:checkpoint_kat).  Eval mode: no
+    batch statistics, no power iteration."""
     from models import gan
     d = np.load(os.path.join(GOLDEN, "gan_checkpoint_kat.npz"))
     G = gan.Generator(GC.make_args(512, 3), 64, symmetric=True, mesh_head=True)
-    G.load_state_dict(torch.load(CKPT, map_location="cpu")["generator_running_avg"], strict=True)
+    G.load_state_dict(GC.checkpoint_standin(gan), strict=True)
     G.cuda().eval()
     with torch.no_grad():
         tex, mesh = G(torch.tensor(d["z"]).cuda(), torch.tensor(d["c"]).cuda())

@@ -1,21 +1,21 @@
-"""The pseudo-ground-truth record format (data/pseudo_gt.py) on the CPU: round trip, dtypes, and — when /root/reference is
-present (authoring container) — that the reference's own dataset class reads our files and mirrors textures identically."""
+"""The pseudo-ground-truth record format (data/pseudo_gt.py) on the CPU: round trip, dtypes, and that the reference's own
+dataset class reads our files and mirrors textures identically (stored golden)."""
 import os
 import sys
 import types
 
 import numpy as np
-import pytest
 import torch
 
-REF = "/root/reference/code"
+from conftest import GOLDEN
+
+sys.path.insert(0, GOLDEN)
+import pseudogt_common as PC          # noqa: E402
 
 
 def _record(seed=0, R=32):
     from data.pseudo_gt import make_record
-    g = torch.Generator().manual_seed(seed)
-    return make_record(torch.randn(3, 32, 32, generator=g) * 0.05, torch.rand(3, R, R, generator=g) * 2 - 1,
-                       (torch.rand(1, R, R, generator=g) > 0.3).float(), torch.rand(4, 16, 16, generator=g) * 2 - 1)
+    return PC.record(make_record, seed, R)
 
 
 def test_round_trip_and_dtypes(tmp_path):
@@ -59,25 +59,18 @@ def test_poses_metadata_round_trip(tmp_path):
     assert torch.equal(d['scale'], s) and torch.equal(d['rotation'], r) and d['path'][3] == "img3.jpg"
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference checkout not present (GPU box)")
-def test_reference_dataset_reads_our_records(tmp_path, monkeypatch):
-    import importlib.util
+def test_reference_dataset_reads_our_records(tmp_path):
+    """tests/golden/pseudogt_dataset_reference.npz (make_golden_reference_state.py): the reference's own
+    AbstractDataset.load_pseudo_ground_truth reading the record this module writes, and its mirror_tex of the texture."""
     from data.pseudo_gt import load_pseudo_ground_truth, mirror_tex, pseudo_gt_dir, save_pseudo_gt
-    spec = importlib.util.spec_from_file_location("ref_abstract_dataset", os.path.join(REF, "data", "abstract_dataset.py"))
-    ref = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ref)
-    rec = _record(seed=3)
+    theirs = np.load(os.path.join(GOLDEN, "pseudogt_dataset_reference.npz"))
     cache = os.path.join(str(tmp_path), "cache", "cub")
-    save_pseudo_gt(pseudo_gt_dir(cache, 32), 0, rec)
-    ds = object.__new__(ref.AbstractDataset)                     # bypass __init__ (it globs the real dataset)
-    ds.args = types.SimpleNamespace(texture_resolution=32)
-    ds.cache_dir = cache
-    theirs = ds.load_pseudo_ground_truth(0)
+    save_pseudo_gt(pseudo_gt_dir(cache, 32), 0, _record(seed=3))
     ours = load_pseudo_ground_truth(cache, 32, 0)
-    assert set(theirs) == set(ours)
+    assert set(theirs.files) == set(ours) | {"mirror_texture"}
     for k in ours:
-        assert torch.equal(theirs[k], ours[k]), k
-    assert torch.equal(ref.AbstractDataset.mirror_tex(ours['texture']), mirror_tex(ours['texture']))
+        assert ours[k].dtype == torch.from_numpy(theirs[k]).dtype and np.array_equal(ours[k].numpy(), theirs[k]), k
+    assert np.array_equal(mirror_tex(ours['texture']).numpy(), theirs["mirror_texture"])
 
 
 def test_export_pipeline_matches_the_reference_export_loop(tmp_path):
