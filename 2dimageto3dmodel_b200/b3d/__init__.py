@@ -76,6 +76,7 @@ _sig("b3d_vertex_pipeline_fwd", _vp, _ll, _ll, _ll, _ll, _i, _i, _vp, _vp, _i, _
 _sig("b3d_vertex_pipeline_bwd", _vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp)
 _sig("b3d_bank_forward", _vp, _vp, _i, _vp, _i, _vp, _i, _vp, _sz, _vp, _i, _vp)
 _sig("b3d_bank_backward", _vp, _vp, _i, _vp, _i, _vp, _vp, _vp, _vp)
+_sig("b3d_bank_up2_grad", _vp, _vp, _i, _i, _i, _vp)
 _sig("b3d_pad_x_fwd", _vp, _vp, _ll, _i, _i, _i, _i, _vp)
 _sig("b3d_pad_x_bwd", _vp, _vp, _ll, _i, _i, _i, _i, _vp)
 _sig("b3d_stem_input_fwd", _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp)
@@ -95,8 +96,8 @@ _sig("b3d_vox_splat_sorted", _vp, _vp, _i, _i, _i, _i, _vp, _vp)
 _sig("b3d_vox_clamp01", _vp, ctypes.c_longlong, _vp)
 _sig("b3d_vox_gather", _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp, _vp)
 _sig("b3d_bn_stats", _vp, _ll, _i, _f, _vp, _vp, _vp, _vp)
-_sig("b3d_cbn_act_fwd", _vp, _vp, _vp, _vp, _i, _i, _vp, _i, _i, _i, _i, _i, _i, _f, _i, _vp)
-_sig("b3d_cbn_act_bwd1", _vp, _vp, _vp, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _i, _i, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _f, _i, _vp)
+_sig("b3d_cbn_act_fwd", _vp, _vp, _vp, _vp, _i, _i, _vp, _i, _i, _i, _i, _i, _i, _f, _i, _i, _vp)
+_sig("b3d_cbn_act_bwd1", _vp, _vp, _vp, _vp, _vp, _i, _i, _vp, _vp, _vp, _vp, _i, _i, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _f, _i, _i, _vp)
 _sig("b3d_cbn_act_bwd2", _vp, _vp, _vp, _vp, _vp, _vp, _vp, _f, _i, _i, _i, _i, _vp)
 _sig("b3d_bn_sums", _vp, _ll, _i, _vp, _vp)
 _sig("b3d_cbn_prepare", _vp, _i, _i, _i, _vp, ctypes.c_double, _f, _f, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, _vp)

@@ -11,6 +11,8 @@ Per layer the bank hands the convolution kernels
   F [T'][Cout][Cin']  tap-major K-major rows (fprop operand; the weight gradient comes back in the same layout),
   D [T'][Cin'][Cout'] its per-tap transpose (input-gradient operand),
 and its backward turns the F-layout gradients into gradients of weight_orig (two launches for the whole network).
+Layers registered as `up2` (3x3 convolutions of a x2 nearest upsample) also get the 16 taps of the four output-parity
+classes, UF [16][Cout][Cin'] and UD [16][Cin'][Cout'] (b3d.conv.upconv_forward / _UpConvBanked).
 """
 import struct
 
@@ -29,19 +31,20 @@ def _r64(v):
 
 class LayerWeights:
     """What one convolution needs from the bank for one forward/backward: wf (autograd output), wd, df (gradient sink)."""
-    __slots__ = ("wf", "wd", "df", "Cout", "Cin", "kh", "kw", "fold", "Cinp", "Coutp", "Tp", "bias")
+    __slots__ = ("wf", "wd", "df", "uf", "ud", "Cout", "Cin", "kh", "kw", "fold", "up2", "Cinp", "Coutp", "Tp", "bias")
 
     def __init__(self, spec):
-        for k in ("Cout", "Cin", "kh", "kw", "fold", "Cinp", "Coutp", "Tp"):
+        for k in ("Cout", "Cin", "kh", "kw", "fold", "up2", "Cinp", "Coutp", "Tp"):
             setattr(self, k, spec[k])
-        self.wf = self.wd = self.df = self.bias = None
+        self.wf = self.wd = self.df = self.uf = self.ud = self.bias = None
 
 
 class WeightBank:
-    def __init__(self, convs, fold=(), no_dgrad=(), round_tf32=True):
+    def __init__(self, convs, fold=(), no_dgrad=(), round_tf32=True, up2=()):
         """convs: ordered {name: conv module} (spectral-normalised modules expose weight_orig / weight_u / weight_v, plain
         ones weight).  fold: names whose kh vertical taps are folded into the channel dimension (thin stems).
-        no_dgrad: names that never need an input gradient (no D layout is written)."""
+        no_dgrad: names that never need an input gradient (no D layout is written).
+        up2: 3x3 layers that also get the class taps of the convolution of a x2 nearest upsample."""
         self.names = list(convs)
         self.mods = [convs[n] for n in self.names]
         # emitted weights rounded to the nearest tf32 value (the tensor cores would otherwise truncate the fp32 words)
@@ -55,7 +58,10 @@ class WeightBank:
             fd = n in fold
             Cinp = _r32(kh * Cin if fd else Cin)
             Tp = kw if fd else kh * kw
-            sp = dict(name=n, sn=sn, Cout=Cout, Cin=Cin, kh=kh, kw=kw, fold=int(fd), Cinp=Cinp, Coutp=_r32(Cout), Tp=Tp,
+            u2 = n in up2
+            if u2 and (fd or (kh, kw) != (3, 3)):
+                raise B3DError(f"bank: {n}: up2 class taps need an unfolded 3x3 layer")
+            sp = dict(name=n, sn=sn, Cout=Cout, Cin=Cin, kh=kh, kw=kw, fold=int(fd), up2=int(u2), Cinp=Cinp, Coutp=_r32(Cout), Tp=Tp,
                       K=Cin * kh * kw, need_d=n not in no_dgrad)
             sp["wf_off"] = off_out
             off_out += _r64(Tp * Cout * Cinp)
@@ -66,6 +72,13 @@ class WeightBank:
             if sp["need_d"]:
                 sp["wd_off"] = off_out
                 off_out += _r64(sp["Tp"] * sp["Cinp"] * sp["Coutp"])
+        for sp in self.specs:
+            sp["uf_off"] = sp["ud_off"] = -1
+            if sp["up2"]:
+                sp["uf_off"] = off_out
+                off_out += _r64(16 * sp["Cout"] * sp["Cinp"])
+                sp["ud_off"] = off_out
+                off_out += _r64(16 * sp["Cinp"] * sp["Coutp"])
         for sp in self.specs:
             sp["u_off"], sp["v_off"], sp["scal_off"] = off_out, off_out + _r64(sp["Cout"]), off_out + _r64(sp["Cout"]) + _r64(sp["K"])
             off_out = sp["scal_off"] + 64
@@ -82,7 +95,7 @@ class WeightBank:
         return [m.weight_orig if sp["sn"] else m.weight for m, sp in zip(self.mods, self.specs)]
 
     def _build(self, device):
-        if lib.b3d_bank_layer_bytes() != 144:
+        if lib.b3d_bank_layer_bytes() != 160:
             raise B3DError("bank: BankLayer record size mismatch between b3d/bank.py and csrc/sn_kernels.cu")
         rec, wtu, wv, emit, dot = [], [], [], [], []
         ptrs = []
@@ -94,10 +107,11 @@ class WeightBank:
                 if t is not None and (not t.is_cuda or t.dtype != torch.float32 or not t.is_contiguous()):
                     raise B3DError(f"bank: {sp['name']}: parameters must be contiguous CUDA fp32 tensors (no CPU fallback)")
             ptrs.append((w.data_ptr(), u.data_ptr() if u is not None else 0, v.data_ptr() if v is not None else 0))
-            rec.append(struct.pack("<3Q9q12i", ptrs[-1][0], ptrs[-1][1], ptrs[-1][2], sp["t_off"], sp["s_off"], sp["wf_off"],
+            rec.append(struct.pack("<3Q11q12i", ptrs[-1][0], ptrs[-1][1], ptrs[-1][2], sp["t_off"], sp["s_off"], sp["wf_off"],
                                    sp["wd_off"], sp["u_off"], sp["v_off"], sp["scal_off"], sp["wf_off"], sp["dw_off"],
+                                   sp["uf_off"], sp["ud_off"],
                                    sp["Cout"], sp["Cin"], sp["kh"], sp["kw"], sp["fold"], sp["Cinp"], sp["Coutp"], sp["Tp"],
-                                   int(sp["sn"]), 0, 0, 0))
+                                   int(sp["sn"]), sp["up2"], 0, 0))
             if sp["sn"]:
                 wtu += [(i, a, b, 0) for a in range(-(-sp["K"] // 256)) for b in range(-(-sp["Cout"] // 64))]
                 wv += [(i, a, 0, 0) for a in range(-(-sp["Cout"] // 8))]
@@ -141,6 +155,8 @@ class WeightBank:
             lw = LayerWeights(sp)
             lw.wf = outs[i]
             lw.wd = outs[n + i] if sp["need_d"] else None
+            if sp["up2"]:
+                lw.uf, lw.ud = outs[2 * n + 1 + 2 * i], outs[2 * n + 2 + 2 * i]
             if need_grad:
                 sz = sp["Tp"] * sp["Cout"] * sp["Cinp"]
                 lw.df = df_flat[sp["wf_off"]: sp["wf_off"] + sz].view(sp["Tp"], sp["Cout"], sp["Cinp"])
@@ -166,9 +182,16 @@ class _BankFn(torch.autograd.Function):
             else:
                 wds.append(out.new_empty(0))
         df = torch.zeros(bank.f_total, device=device, dtype=torch.float32) if need_grad else out.new_empty(0)
+        ups = []                                            # (UF, UD) per layer (empty for layers without up2)
+        for sp in bank.specs:
+            if sp["up2"]:
+                ups.append(out[sp["uf_off"]: sp["uf_off"] + 16 * sp["Cout"] * sp["Cinp"]].view(16, sp["Cout"], sp["Cinp"]))
+                ups.append(out[sp["ud_off"]: sp["ud_off"] + 16 * sp["Cinp"] * sp["Coutp"]].view(16, sp["Cinp"], sp["Coutp"]))
+            else:
+                ups += [out.new_empty(0), out.new_empty(0)]
         ctx.bank, ctx.out, ctx.df = bank, out, df
-        ctx.mark_non_differentiable(*wds, df)
-        return (*wfs, *wds, df)
+        ctx.mark_non_differentiable(*wds, df, *ups)
+        return (*wfs, *wds, df, *ups)
 
     @staticmethod
     def backward(ctx, *grads):

@@ -501,3 +501,79 @@ def conv2d_banked(x_nchw, lw, pad_y=0, stride=1, leaky=1.0, pad_out=0, pad_mode=
     y = _ConvBanked.apply(x, lw.wf, lw.bias, lw, int(pad_y), int(stride), float(leaky), int(pad_out), int(pad_mode), int(x_crop), stats,
                           fold_raw, link_in, link_out)
     return y.permute(0, 3, 1, 2)
+
+
+# ------------------------------------------------------------------------------------------------------------------
+# Up-convolution: conv3x3(up2(x)) (zero padding in y, x padding already in the input) run on x itself.  Every 2x2 block of
+# the nearest-upsampled tensor holds one value, so output pixel (2i+a, 2j+b) is a 2x2 convolution of x with the class taps
+# K_ab = A_a W A_b^T (A_0 = [[1,0,0],[0,1,1]], A_1 = [[1,1,0],[0,0,1]]; the bank's `up2` layouts): 4 MACs per output pixel
+# and input channel instead of 9.  With x replicate-padded by one column, up2 of it is the replicate-padded up2(x), so the
+# padded low-resolution tensor stands in for the padded upsampled one.
+# ------------------------------------------------------------------------------------------------------------------
+def upconv_taps():
+    """Tap lists of the up-convolution, tap t = ((a*2 + b)*2 + u)*2 + v (class (a, b), class tap (u, v)), in the pixel
+    coordinates of b3d_conv2d_tf32 (pure index arithmetic, unit-tested on the CPU):
+      forward  Y[2i+a, 2j+b]  += K_ab[u][v] . Xp[i + a-1+u, j + b+v]       (Xp: x padded by one column, zero rows outside)
+      dgrad    dXp[i, j]      += K_ab[u][v]^T . dY[2i + 2-a-2u, 2j - b-2v]  (input stride 2, zeros outside dY)
+    The weight gradient runs b3d_conv2d_wgrad_tf32 with the operands swapped (Xp as "dy", dY as the stride-2 "x", kh = kw =
+    4, pad_y = 1, x_off = -3): its tap (R, S) = (3-a-2u, 3-b-2v) is dK_ab[u][v]^T.  -> (classes, fdy, fdx, ddy, ddx)."""
+    classes = [(a, b) for a in range(2) for b in range(2)]
+    t = [(a, b, u, v) for a, b in classes for u in range(2) for v in range(2)]
+    return (classes, [a - 1 + u for a, b, u, v in t], [b + v for a, b, u, v in t], [2 - a - 2 * u for a, b, u, v in t],
+            [-b - 2 * v for a, b, u, v in t])
+
+
+_UPCONV = upconv_taps()
+
+
+class _UpConvBanked(torch.autograd.Function):
+    @staticmethod
+    def forward(ctx, x, wf, lw, stats):
+        """x [N,H,W+2,Cin] (replicate-padded by one column) -> conv3x3(up2(x)) [N,2H,2W,Cout]; stats as conv2d_banked's."""
+        x = dev(x.detach(), "x")
+        N, H, Wp, Cin = x.shape
+        if not lw.up2 or Cin != lw.Cinp or lw.Cout % 32:
+            raise B3DError("upconv: the layer needs the bank's up2 class taps, Cin' input channels and Cout % 32 == 0")
+        W, Cout = Wp - 2, lw.Cout
+        classes, fdy, fdx, _, _ = _UPCONV
+        out = torch.empty(N, 2 * H, 2 * W, Cout, device=x.device, dtype=torch.float32)
+        opts = _ConvOpts(None, 1.0, 0, 0, 4)
+        for i, (a, b) in enumerate(classes):
+            opts.class_ooy[i], opts.class_oox[i] = a, b
+        check(_conv_call(lib.b3d_conv2d_tf32, ptr(x), ptr(dev(lw.uf, "weight")), None, ptr(out), N, H, Wp, Cin, H, W, Cout, 16,
+                         _ints(fdy), _ints(fdx), 1, 1, 2 * H, 2 * W, Cout, 2, 2, 0, 0, 1.0, 0, None, 0, ptr(stats), 0, 0,
+                         ctypes.cast(ctypes.pointer(opts), ctypes.c_void_p), stream_ptr(x)))
+        ctx.save_for_backward(x)
+        ctx.lw = lw
+        return out
+
+    @staticmethod
+    def backward(ctx, gy):
+        x, = ctx.saved_tensors
+        lw = ctx.lw
+        N, H, Wp, Cin = x.shape
+        Cout = lw.Cout
+        gy = dev(gy, "grad_output")
+        st = stream_ptr(gy)
+        _, _, _, ddy, ddx = _UPCONV
+        gx = gw = None
+        if ctx.needs_input_grad[0]:
+            gx = torch.empty(N, H, Wp, Cin, device=gy.device, dtype=torch.float32)
+            check(_conv_call(lib.b3d_conv2d_tf32, ptr(gy), ptr(dev(lw.ud, "weight")), None, ptr(gx), N, 2 * H, 2 * (Wp - 2), Cout, H, Wp,
+                             Cin, 16, _ints(ddy), _ints(ddx), 2, 2, H, Wp, Cin, 1, 1, 0, 0, 1.0, 0, None, 0, None, 0, 0, None, st))
+        if ctx.needs_input_grad[1]:
+            gw = lw.df                                                 # the bank's 3x3 gradient sink (zeroed by the bank)
+            if gw is None:
+                raise B3DError("upconv: weight gradient requested but the bank was run without gradients")
+            dk = torch.zeros(16, Cin, Cout, device=gy.device, dtype=torch.float32)
+            check(_conv_call(lib.b3d_conv2d_wgrad_tf32, ptr(x), ptr(gy), ptr(dk), N, 2 * H, 2 * (Wp - 2), Cout, H, Wp, Cin, 4, 4, 1, 2,
+                             -3, 1, 0, 0, st))
+            check(lib.b3d_bank_up2_grad(ptr(dk), ptr(gw), Cout, lw.Cin, lw.Cinp, st))
+        return gx, gw, None, None
+
+
+def upconv_banked(x_nchw, lw, stats=None):
+    """conv2d_banked(up2(x), lw, pad_y=1) for a 3x3 layer the bank serves as `up2`, with x the replicate-padded input of the
+    upsample (logically NCHW, channels-last) — the x4 tensor is never written."""
+    y = _UpConvBanked.apply(x_nchw.permute(0, 2, 3, 1), lw.wf, lw, stats)
+    return y.permute(0, 3, 1, 2)

@@ -157,11 +157,12 @@ class BNAffine(CBNBatch):
 
 class _CBNActPad(torch.autograd.Function):
     """y [N,H,W,C] (conv output, NHWC) -> out [N, up*H, up*W + 2*pad, C]; gb = CBNBatch.gb (gamma / beta of this layer at
-    column offsets goff / boff).  `skip` (optional) [N,H,Ws,C] read at pixel offset skip_off.  Statistics, running buffers
+    column offsets goff / boff).  `skip` (optional) [N,H,Ws,C] read at pixel offset skip_off; skip_half: [N,H/2,Ws,C] read at
+    (y/2, x/2).  Statistics, running buffers
     and the per-sample affine come from one b3d_cbn_prepare launch (modes: 0 eval, 1 batch statistics, 2 SyncBN)."""
 
     @staticmethod
-    def forward(ctx, y, gb, cb, key, bn, skip, skip_off, up, pad, post_leaky, sums_in=None, slope=0.2):
+    def forward(ctx, y, gb, cb, key, bn, skip, skip_off, up, pad, post_leaky, sums_in=None, slope=0.2, skip_half=0):
         y = dev(y.detach(), "y")
         N, H, W, C = y.shape
         gbd = dev(gb.detach(), "gamma/beta")
@@ -206,18 +207,18 @@ class _CBNActPad(torch.autograd.Function):
         pitch = sk.shape[2] if sk is not None else 0
         out = torch.empty(N, up * H, up * W + 2 * pad, C, device=y.device, dtype=torch.float32)
         check(lib.b3d_cbn_act_fwd(ptr(y), ptr(scale), ptr(shift), ptr(sk), pitch, skip_off, ptr(out), N, H, W, C, up, pad, float(slope),
-                                  int(post_leaky), st))
+                                  int(post_leaky), int(skip_half), st))
         ctx.save_for_backward(y, gt, scale, shift, mean, invstd, sk if sk is not None else torch.empty(0))
         ctx.cb, ctx.key = cb, key
         ctx.cfg = (skip_off, up, pad, post_leaky, mode != 0, sync, count, sk is not None, skip.shape if skip is not None else None,
-                   P, goff, boff, float(slope))
+                   P, goff, boff, float(slope), int(skip_half))
         ctx.peers = peers
         return out
 
     @staticmethod
     def backward(ctx, gout):
         y, gt, scale, shift, mean, invstd, sk = ctx.saved_tensors
-        skip_off, up, pad, post_leaky, batch_stats, sync, count, has_skip, skip_shape, P, goff, boff, slope = ctx.cfg
+        skip_off, up, pad, post_leaky, batch_stats, sync, count, has_skip, skip_shape, P, goff, boff, slope, skip_half = ctx.cfg
         cb = ctx.cb
         N, H, W, C = y.shape
         gout = dev(gout, "grad")
@@ -226,14 +227,15 @@ class _CBNActPad(torch.autograd.Function):
         gskip, gpitch = None, 0
         if has_skip and ctx.needs_input_grad[5]:
             gpitch = skip_shape[2]
-            gskip = torch.zeros(skip_shape, device=y.device) if gpitch != W else torch.empty(skip_shape, device=y.device)
+            dense = gpitch == W >> skip_half
+            gskip = torch.empty(skip_shape, device=y.device) if dense else torch.zeros(skip_shape, device=y.device)
         want_gb = ctx.needs_input_grad[1]
         sink = cb.grad_sink(N) if want_gb else torch.empty(N, P, device=y.device)
         s1 = ctypes.c_void_p(sink.data_ptr() + 4 * boff)        # d beta  = sum ga
         s2 = ctypes.c_void_p(sink.data_ptr() + 4 * goff)        # d gamma = sum ga * xhat
         check(lib.b3d_cbn_act_bwd1(ptr(gout), ptr(y), ptr(scale), ptr(shift), ptr(sk) if has_skip else None,
                                    sk.shape[2] if has_skip else 0, skip_off, ptr(mean), ptr(invstd), ptr(ga), ptr(gskip), gpitch,
-                                   skip_off, s1, s2, P, N, H, W, C, up, pad, slope, int(post_leaky), st))
+                                   skip_off, s1, s2, P, N, H, W, C, up, pad, slope, int(post_leaky), skip_half, st))
         inv_m = 0.0
         if batch_stats:
             red = torch.empty(2 * C, device=y.device, dtype=torch.float32)
@@ -258,7 +260,7 @@ class _CBNActPad(torch.autograd.Function):
                 if cb.done != cb.n_layers:
                     raise RuntimeError(f"CBNBatch: {cb.done} of {cb.n_layers} layers ran their backward before the first layer's")
                 ggb = sink.sum(dim=0, keepdim=True) if cb.shared else sink
-        return ga, ggb, None, None, None, gskip, None, None, None, None, None, None
+        return ga, ggb, None, None, None, gskip, None, None, None, None, None, None, None
 
 
 _BN_STATS_IMPL = os.environ.get("B3D_BN_STATS", "torch")
@@ -291,8 +293,9 @@ def bn_act_pad(y_nchw, bn, skip_nchw=None, skip_off=0, up=1, pad=1, post_relu=Fa
     return out.permute(0, 3, 1, 2)
 
 
-def cbn_act_pad(y_nchw, cbn, z, skip_nchw=None, skip_off=0, up=1, pad=1, post_leaky=False, cb=None, sums=None):
+def cbn_act_pad(y_nchw, cbn, z, skip_nchw=None, skip_off=0, up=1, pad=1, post_leaky=False, cb=None, sums=None, skip_half=False):
     """ConditionalBatchNorm2d(y, z) -> LeakyReLU(0.2) [-> + skip] [-> LeakyReLU] [-> x2 upsample] -> replicate pad, fused.
+    skip_half: the skip is at half y's resolution and is added as its x2 nearest upsample.
     `cbn` is a models.gan.ConditionalBatchNorm2d whose .norm is a (Synchronized)BatchNorm2d without affine; statistics and
     running buffers follow F.batch_norm (single process) or the reference's SyncBN formulas (torch.distributed).
     cb: the forward's CBNBatch (gamma / beta of all layers from one GEMM); None = a one-layer batch built here."""
@@ -303,5 +306,6 @@ def cbn_act_pad(y_nchw, cbn, z, skip_nchw=None, skip_off=0, up=1, pad=1, post_le
     if C % 4 or 256 % (C // 4):
         raise B3DError(f"cbn_act_pad: C={C} must be 4 * a divisor of 256")
     skip = skip_nchw.permute(0, 2, 3, 1) if skip_nchw is not None else None
-    out = _CBNActPad.apply(y, cb.gb, cb, id(cbn), cbn.norm, skip, int(skip_off), int(up), int(pad), bool(post_leaky), sums)
+    out = _CBNActPad.apply(y, cb.gb, cb, id(cbn), cbn.norm, skip, int(skip_off), int(up), int(pad), bool(post_leaky), sums, 0.2,
+                           int(bool(skip_half)))
     return out.permute(0, 3, 1, 2)

@@ -705,7 +705,13 @@ struct CbnGeom {
     int skip_pitch, skip_off;    // skip pixel (y,x) lives at row (y*skip_pitch + x + skip_off); pitch 0 = no skip
     float slope;                 // LeakyReLU slope of the first activation
     int post_leaky;              // apply LeakyReLU again after the residual add (blk6 / mesh head)
+    int skip_half;               // the skip is at half resolution: pixel (y,x) reads skip pixel (y/2, x/2) of [N,H/2,..]
 };
+
+__device__ __forceinline__ long long skip_pixel(const CbnGeom& g, int n, int ys, int xs) {
+    const int sh = g.skip_half;
+    return ((long long)n * (g.H >> sh) + (ys >> sh)) * g.skip_pitch + (xs >> sh) + g.skip_off;
+}
 
 __device__ __forceinline__ float lk(float v, float s) { return v >= 0.f ? v : v * s; }
 
@@ -730,7 +736,7 @@ cbn_act_fwd_kernel(const float4* __restrict__ y, const float4* __restrict__ scal
         float4 o = make_float4(lk(fmaf(v.x, sc.x, sh.x), g.slope), lk(fmaf(v.y, sc.y, sh.y), g.slope),
                                lk(fmaf(v.z, sc.z, sh.z), g.slope), lk(fmaf(v.w, sc.w, sh.w), g.slope));
         if (g.skip_pitch) {
-            const float4 k = __ldg(skip + (((long long)n * g.H + ys) * g.skip_pitch + xs + g.skip_off) * g.C4 + c);
+            const float4 k = __ldg(skip + skip_pixel(g, n, ys, xs) * g.C4 + c);
             o.x += k.x; o.y += k.y; o.z += k.z; o.w += k.w;
         }
         if (g.post_leaky) o = make_float4(lk(o.x, g.slope), lk(o.y, g.slope), lk(o.z, g.slope), lk(o.w, g.slope));
@@ -751,7 +757,7 @@ cbn_act_fwd_rows_kernel(const float4* __restrict__ y, const float4* __restrict__
         const int ys = yo / g.up;
         const float4 sc = __ldg(scale + (long long)n * g.C4 + c), sh = __ldg(shift + (long long)n * g.C4 + c);
         const float4* yrow = y + (((long long)n * g.H + ys) * g.W) * g.C4 + c;
-        const float4* srow = g.skip_pitch ? skip + (((long long)n * g.H + ys) * g.skip_pitch + g.skip_off) * g.C4 + c : nullptr;
+        const float4* srow = g.skip_pitch ? skip + skip_pixel(g, n, ys, 0) * g.C4 + c : nullptr;
         float4* orow = out + (long long)row * Wo * g.C4 + c;
         constexpr int U = 4;                                 // independent pixels in flight per thread
         for (int xb = px0; xb < Wo; xb += U * PPB) {
@@ -764,7 +770,7 @@ cbn_act_fwd_rows_kernel(const float4* __restrict__ y, const float4* __restrict__
                 xs = xs < 0 ? 0 : (xs >= Wu ? Wu - 1 : xs);
                 xs = g.up == 2 ? xs >> 1 : xs;
                 v[u] = __ldg(yrow + (long long)xs * g.C4);
-                if (srow) k[u] = __ldg(srow + (long long)xs * g.C4);
+                if (srow) k[u] = __ldg(srow + (long long)(xs >> g.skip_half) * g.C4);
             }
 #pragma unroll
             for (int u = 0; u < U; ++u) {
@@ -783,6 +789,8 @@ cbn_act_fwd_rows_kernel(const float4* __restrict__ y, const float4* __restrict__
 // Backward pass 1.  Per input pixel: gather the gradient of its up x up children (+ the replicate-pad columns), undo the
 // activations, write ga = d/d(pre-activation) and (optionally) gskip; accumulate S1[n,c] = sum ga, S2[n,c] = sum ga * xhat
 // with xhat = (y - mean) * inv_std.  One CTA walks `rows_per_cta` image rows of one sample, threads own channel quads.
+// Half-resolution skip: a thread owns a skip pixel and its 2x2 input pixels, and writes their summed skip gradient once
+// (no atomics: the sum order is fixed, the step repeats bit for bit).
 __global__ void __launch_bounds__(NT)
 cbn_act_bwd1_kernel(const float4* __restrict__ gout, const float4* __restrict__ y, const float4* __restrict__ scale,
                     const float4* __restrict__ shift, const float4* __restrict__ skip, const float4* __restrict__ mean,
@@ -791,41 +799,47 @@ cbn_act_bwd1_kernel(const float4* __restrict__ gout, const float4* __restrict__ 
     const int n = blockIdx.y;
     const int y0 = blockIdx.x * rows_per_cta, y1 = min(y0 + rows_per_cta, g.H);
     const int Wo = g.up * g.W + 2 * g.pad;
+    const int sh = g.skip_half, Wk = g.W >> sh;               // pixels owned per thread: (1 << sh) x (1 << sh)
     for (int c = threadIdx.x % g.C4, lane_px = threadIdx.x / g.C4, px_step = NT / g.C4; c < g.C4; c += g.C4) {
-        const float4 sc = __ldg(scale + (long long)n * g.C4 + c), sh = __ldg(shift + (long long)n * g.C4 + c);
+        const float4 sc = __ldg(scale + (long long)n * g.C4 + c), sh4 = __ldg(shift + (long long)n * g.C4 + c);
         const float4 mu = __ldg(mean + c), is = __ldg(invstd + c);
         float4 a1 = make_float4(0.f, 0.f, 0.f, 0.f), a2 = a1;
-        for (int p = y0 * g.W + lane_px; p < y1 * g.W; p += px_step) {
-            const int ys = p / g.W, xs = p % g.W;
-            float4 s = make_float4(0.f, 0.f, 0.f, 0.f);
-            for (int i = 0; i < g.up; ++i) {
-                const float4* row = gout + (((long long)n * g.up * g.H + g.up * ys + i) * Wo) * g.C4 + c;
-                int lo = g.up * xs + g.pad, hi = lo + g.up;          // children columns [lo, hi)
-                if (xs == 0) lo = 0;                                  // left pad columns replicate column 0
-                if (xs == g.W - 1) hi = Wo;                           // right pad columns replicate the last column
-                for (int xo = lo; xo < hi; ++xo) {
-                    const float4 v = __ldg(row + (long long)xo * g.C4);
-                    s.x += v.x; s.y += v.y; s.z += v.z; s.w += v.w;
+        for (int p = (y0 >> sh) * Wk + lane_px; p < (y1 >> sh) * Wk; p += px_step) {
+            const int yk = p / Wk, xk = p % Wk;
+            float4 gs = make_float4(0.f, 0.f, 0.f, 0.f);
+            for (int q = 0; q < (1 << (2 * sh)); ++q) {
+                const int ys = (yk << sh) + (q >> 1) * sh, xs = (xk << sh) + (q & 1) * sh;
+                float4 s = make_float4(0.f, 0.f, 0.f, 0.f);
+                for (int i = 0; i < g.up; ++i) {
+                    const float4* row = gout + (((long long)n * g.up * g.H + g.up * ys + i) * Wo) * g.C4 + c;
+                    int lo = g.up * xs + g.pad, hi = lo + g.up;          // children columns [lo, hi)
+                    if (xs == 0) lo = 0;                                  // left pad columns replicate column 0
+                    if (xs == g.W - 1) hi = Wo;                           // right pad columns replicate the last column
+                    for (int xo = lo; xo < hi; ++xo) {
+                        const float4 v = __ldg(row + (long long)xo * g.C4);
+                        s.x += v.x; s.y += v.y; s.z += v.z; s.w += v.w;
+                    }
                 }
+                const long long idx = (((long long)n * g.H + ys) * g.W + xs) * g.C4 + c;
+                const float4 v = __ldg(y + idx);
+                const float4 pre = make_float4(fmaf(v.x, sc.x, sh4.x), fmaf(v.y, sc.y, sh4.y), fmaf(v.z, sc.z, sh4.z), fmaf(v.w, sc.w, sh4.w));
+                if (g.post_leaky) {                                       // sign of (leaky(pre) + skip)
+                    float4 k = make_float4(0.f, 0.f, 0.f, 0.f);
+                    if (g.skip_pitch) k = __ldg(skip + skip_pixel(g, n, ys, xs) * g.C4 + c);
+                    s.x = (lk(pre.x, g.slope) + k.x) >= 0.f ? s.x : s.x * g.slope;
+                    s.y = (lk(pre.y, g.slope) + k.y) >= 0.f ? s.y : s.y * g.slope;
+                    s.z = (lk(pre.z, g.slope) + k.z) >= 0.f ? s.z : s.z * g.slope;
+                    s.w = (lk(pre.w, g.slope) + k.w) >= 0.f ? s.w : s.w * g.slope;
+                }
+                gs.x += s.x; gs.y += s.y; gs.z += s.z; gs.w += s.w;
+                const float4 a = make_float4(pre.x >= 0.f ? s.x : s.x * g.slope, pre.y >= 0.f ? s.y : s.y * g.slope,
+                                             pre.z >= 0.f ? s.z : s.z * g.slope, pre.w >= 0.f ? s.w : s.w * g.slope);
+                ga[idx] = a;
+                a1.x += a.x; a1.y += a.y; a1.z += a.z; a1.w += a.w;
+                a2.x = fmaf(a.x, (v.x - mu.x) * is.x, a2.x); a2.y = fmaf(a.y, (v.y - mu.y) * is.y, a2.y);
+                a2.z = fmaf(a.z, (v.z - mu.z) * is.z, a2.z); a2.w = fmaf(a.w, (v.w - mu.w) * is.w, a2.w);
             }
-            const long long idx = (((long long)n * g.H + ys) * g.W + xs) * g.C4 + c;
-            const float4 v = __ldg(y + idx);
-            const float4 pre = make_float4(fmaf(v.x, sc.x, sh.x), fmaf(v.y, sc.y, sh.y), fmaf(v.z, sc.z, sh.z), fmaf(v.w, sc.w, sh.w));
-            if (g.post_leaky) {                                       // sign of (leaky(pre) + skip)
-                float4 k = make_float4(0.f, 0.f, 0.f, 0.f);
-                if (g.skip_pitch) k = __ldg(skip + (((long long)n * g.H + ys) * g.skip_pitch + xs + g.skip_off) * g.C4 + c);
-                s.x = (lk(pre.x, g.slope) + k.x) >= 0.f ? s.x : s.x * g.slope;
-                s.y = (lk(pre.y, g.slope) + k.y) >= 0.f ? s.y : s.y * g.slope;
-                s.z = (lk(pre.z, g.slope) + k.z) >= 0.f ? s.z : s.z * g.slope;
-                s.w = (lk(pre.w, g.slope) + k.w) >= 0.f ? s.w : s.w * g.slope;
-            }
-            if (gskip) gskip[(((long long)n * g.H + ys) * gskip_pitch + xs + gskip_off) * g.C4 + c] = s;
-            const float4 a = make_float4(pre.x >= 0.f ? s.x : s.x * g.slope, pre.y >= 0.f ? s.y : s.y * g.slope,
-                                         pre.z >= 0.f ? s.z : s.z * g.slope, pre.w >= 0.f ? s.w : s.w * g.slope);
-            ga[idx] = a;
-            a1.x += a.x; a1.y += a.y; a1.z += a.z; a1.w += a.w;
-            a2.x = fmaf(a.x, (v.x - mu.x) * is.x, a2.x); a2.y = fmaf(a.y, (v.y - mu.y) * is.y, a2.y);
-            a2.z = fmaf(a.z, (v.z - mu.z) * is.z, a2.z); a2.w = fmaf(a.w, (v.w - mu.w) * is.w, a2.w);
+            if (gskip) gskip[(((long long)n * (g.H >> sh) + yk) * gskip_pitch + xk + gskip_off) * g.C4 + c] = gs;
         }
         float* s1 = S1 + (long long)n * s_pitch + c * 4;
         float* s2 = S2 + (long long)n * s_pitch + c * 4;
@@ -855,12 +869,14 @@ cbn_act_bwd2_kernel(float4* __restrict__ ga, const float4* __restrict__ y, const
 
 extern "C" {
 int b3d_cbn_act_fwd(const float* y, const float* scale, const float* shift, const float* skip, int skip_pitch, int skip_off,
-                    float* out, int N, int H, int W, int C, int up, int pad, float slope, int post_leaky, void* stream) {
+                    float* out, int N, int H, int W, int C, int up, int pad, float slope, int post_leaky, int skip_half,
+                    void* stream) {
     B3D_REQUIRE(N >= 0 && H > 0 && W > 0 && C > 0 && C % 4 == 0 && (up == 1 || up == 2) && pad >= 0, B3D_EINVAL,
                 "b3d_cbn_act_fwd: bad arguments");
+    B3D_REQUIRE(!skip_half || (skip_half == 1 && H % 2 == 0 && W % 2 == 0), B3D_EINVAL, "b3d_cbn_act_fwd: a half-resolution skip needs even H, W");
     if (N == 0) return B3D_OK;
     B3D_REQUIRE(y && scale && shift && out && (skip != nullptr) == (skip_pitch != 0), B3D_EINVAL, "b3d_cbn_act_fwd: null pointer");
-    CbnGeom g{N, H, W, C / 4, up, pad, skip_pitch, skip_off, slope, post_leaky};
+    CbnGeom g{N, H, W, C / 4, up, pad, skip_pitch, skip_off, slope, post_leaky, skip_half};
     const long long total = (long long)N * up * H * (up * W + 2 * pad) * (C / 4);
     if (g.C4 <= NT && NT % g.C4 == 0 && (up == 1 || up == 2)) {
         const int rows = N * up * H;
@@ -879,7 +895,8 @@ int b3d_cbn_act_fwd(const float* y, const float* scale, const float* shift, cons
 int b3d_cbn_act_bwd1(const float* gout, const float* y, const float* scale, const float* shift, const float* skip, int skip_pitch,
                      int skip_off, const float* mean, const float* invstd, float* ga, float* gskip, int gskip_pitch, int gskip_off,
                      float* S1, float* S2, int s_pitch, int N, int H, int W, int C, int up, int pad, float slope, int post_leaky,
-                     void* stream) {
+                     int skip_half, void* stream) {
+    B3D_REQUIRE(!skip_half || (skip_half == 1 && H % 2 == 0 && W % 2 == 0), B3D_EINVAL, "b3d_cbn_act_bwd1: a half-resolution skip needs even H, W");
     B3D_REQUIRE(N >= 0 && H > 0 && W > 0 && C > 0 && C % 4 == 0 && C / 4 <= NT && NT % (C / 4) == 0 && (up == 1 || up == 2), B3D_EINVAL,
                 "b3d_cbn_act_bwd1: bad arguments (C/4 must divide %d)", NT);
     if (N == 0) return B3D_OK;
@@ -888,10 +905,11 @@ int b3d_cbn_act_bwd1(const float* gout, const float* y, const float* scale, cons
     B3D_REQUIRE(s_pitch >= C && s_pitch % 4 == 0, B3D_EINVAL, "b3d_cbn_act_bwd1: S pitch %d must be >= C and a multiple of 4", s_pitch);
     B3D_CUDA_OK(cudaMemset2DAsync(S1, sizeof(float) * (size_t)s_pitch, 0, sizeof(float) * (size_t)C, (size_t)N, st));
     B3D_CUDA_OK(cudaMemset2DAsync(S2, sizeof(float) * (size_t)s_pitch, 0, sizeof(float) * (size_t)C, (size_t)N, st));
-    CbnGeom g{N, H, W, C / 4, up, pad, skip_pitch, skip_off, slope, post_leaky};
-    // enough CTAs to fill the GPU a few times, each with >= 1 row
+    CbnGeom g{N, H, W, C / 4, up, pad, skip_pitch, skip_off, slope, post_leaky, skip_half};
+    // enough CTAs to fill the GPU a few times, each with >= 1 row (an even number with a half-resolution skip)
     int rows = (int)(((long long)N * H + 148 * 8 - 1) / (148 * 8));
     rows = rows < 1 ? 1 : rows;
+    rows += rows & skip_half;
     dim3 grid(b3d::ceil_div(H, rows), N);
     cbn_act_bwd1_kernel<<<grid, NT, 0, st>>>((const float4*)gout, (const float4*)y, (const float4*)scale, (const float4*)shift,
                                             (const float4*)skip, (const float4*)mean, (const float4*)invstd, (float4*)ga,

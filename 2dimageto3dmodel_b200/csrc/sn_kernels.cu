@@ -15,6 +15,11 @@
 // plain (fold = 0): T' = kh*kw, Cin' = Cin rounded up to 32 (zero filled);
 // folded stems (fold = 1, discriminator conv1 with 8 / 11 input channels): the kh vertical taps live in the channel
 // dimension, T' = kw, Cin' = kh*Cin rounded up to 32, F[s][co][r*Cin + c] = W[co][c][r][s] (b3d/conv.py:fold_kh_weight).
+// up2 layers (3x3 convolutions whose input is a x2 nearest upsample, read before the upsample): ALSO the 16 taps of the four
+// output-parity classes, UF [16][Cout][Cin'] and UD [16][Cin'][Cout'], tap ((a*2 + b)*2 + u)*2 + v = K_ab[u][v] with
+// K_ab = A_a W A_b^T, A_0 = [[1,0,0],[0,1,1]], A_1 = [[1,1,0],[0,0,1]]: output pixel (2i+a, 2j+b) of conv3x3(up2(x)) is the
+// 2x2 convolution K_ab of x at rows i+a-1+u, columns j+b+v (b3d/conv.py upconv_taps).  Summed in fp32 from W / sigma, then
+// rounded to tf32 once.  The weight gradient still arrives in the 3x3 F layout (b3d_bank_up2_grad applies the adjoint).
 //
 // Launch structure: every kernel walks a host-built list of (layer, chunk) work items, one CTA each, so all layers of a
 // network share the launches: zero scratch (memset) -> W^T u -> W v -> emit;  backward: <dF, F> -> dW.
@@ -41,10 +46,35 @@ struct alignas(16) BankLayer {
     long long scal_off;  // out: [2] = (sigma, <dF, F> accumulator)
     long long df_off;    // backward in : gradient in F layout (offset into the dF buffer = wf_off's numbering)
     long long dw_off;    // backward out: gradient in weight_orig layout
+    long long uf_off;    // out: up2 class taps, UF layout, or -1
+    long long ud_off;    // out: up2 class taps, UD layout, or -1
     int Cout, Cin, kh, kw;
     int fold, Cinp, Coutp, Tp;
-    int sn, pad0, pad1, pad2;
+    int sn, up2, pad1, pad2;
 };
+
+// the 16 class taps of a 3x3 kernel w[r][s] (see the layout comment at the top)
+__device__ __forceinline__ void up2_taps(const float w[9], float k[16]) {
+    float rw[2][2][3];                                  // rw[a][u][s] = sum_r A_a[u][r] w[r][s]
+#pragma unroll
+    for (int s = 0; s < 3; ++s) {
+        rw[0][0][s] = w[s];
+        rw[0][1][s] = w[3 + s] + w[6 + s];
+        rw[1][0][s] = w[s] + w[3 + s];
+        rw[1][1][s] = w[6 + s];
+    }
+#pragma unroll
+    for (int a = 0; a < 2; ++a)
+#pragma unroll
+        for (int u = 0; u < 2; ++u) {
+            const float* q = rw[a][u];
+            const float c[2][2] = {{q[0], q[1] + q[2]}, {q[0] + q[1], q[2]}};      // c[b][v] = sum_s A_b[v][s] q[s]
+#pragma unroll
+            for (int b = 0; b < 2; ++b)
+#pragma unroll
+                for (int v = 0; v < 2; ++v) k[((a * 2 + b) * 2 + u) * 2 + v] = c[b][v];
+        }
+}
 
 struct Item { int layer, a, b, c; };
 
@@ -183,6 +213,30 @@ bank_emit_kernel(const BankLayer* __restrict__ layers, const Item* __restrict__ 
             outb[L.wf_off + ((size_t)tp * L.Cout + co) * L.Cinp + ci] = val;
         }
     }
+    if (L.up2) {
+        // UF: lanes along ci' (coalesced stores)
+        for (int e = threadIdx.x; e < 32 * 32; e += NT) {
+            const int ci = ci0 + (e & 31), co = co0 + (e >> 5);
+            if (co >= L.Cout || ci >= L.Cinp) continue;
+            float w[9], k[16];
+#pragma unroll
+            for (int t = 0; t < 9; ++t) w[t] = ci < L.Cin ? __ldg(L.w + (co * L.Cin + ci) * 9 + t) * rs : 0.f;
+            up2_taps(w, k);
+#pragma unroll
+            for (int t = 0; t < 16; ++t) outb[L.uf_off + ((size_t)t * L.Cout + co) * L.Cinp + ci] = tf32_rna(k[t], round_tf32);
+        }
+        // UD: lanes along co' (coalesced stores); rows co >= Cout are zero
+        for (int e = threadIdx.x; e < 32 * 32; e += NT) {
+            const int co = co0 + (e & 31), ci = ci0 + (e >> 5);
+            if (co >= L.Coutp || ci >= L.Cinp) continue;
+            float w[9], k[16];
+#pragma unroll
+            for (int t = 0; t < 9; ++t) w[t] = (ci < L.Cin && co < L.Cout) ? __ldg(L.w + (co * L.Cin + ci) * 9 + t) * rs : 0.f;
+            up2_taps(w, k);
+#pragma unroll
+            for (int t = 0; t < 16; ++t) outb[L.ud_off + ((size_t)t * L.Cinp + ci) * L.Coutp + co] = tf32_rna(k[t], round_tf32);
+        }
+    }
     if (L.wd_off < 0) return;
     // D: lanes along co' (coalesced stores); rows co >= Cout are zero
     const int cop0 = it.a * 32;
@@ -254,6 +308,28 @@ bank_bwd_emit_kernel(const BankLayer* __restrict__ layers, const Item* __restric
     }
 }
 
+// Adjoint of the up2 class taps: dF[r*3 + s][co][ci] += sum_{R in {3-r, 2-r}} sum_{S in {3-s, 2-s}} dk[R*4 + S][ci][co], with dk
+// the weight gradient of the up-convolution in b3d_conv2d_wgrad_tf32's tap-major layout [4x4][Cin][Cout] (tap (R, S) =
+// class (a, b), tap (u, v) at R = 3 - a - 2u, S = 3 - b - 2v; b3d/conv.py _UpConvBanked).  One thread per (ci, co).
+__global__ void __launch_bounds__(NT)
+bank_up2_grad_kernel(const float* __restrict__ dk, float* __restrict__ df, int Cout, int Cin, int Cinp) {
+    const long long e = (long long)blockIdx.x * NT + threadIdx.x;
+    if (e >= (long long)Cin * Cout) return;
+    const int co = (int)(e % Cout), ci = (int)(e / Cout);
+    const size_t plane = (size_t)Cin * Cout;
+    float g[16];
+#pragma unroll
+    for (int t = 0; t < 16; ++t) g[t] = __ldg(dk + t * plane + e);
+#pragma unroll
+    for (int r = 0; r < 3; ++r)
+#pragma unroll
+        for (int s = 0; s < 3; ++s) {
+            const int R = 3 - r, S = 3 - s;
+            const float v = (g[R * 4 + S] + g[R * 4 + S - 1]) + (g[(R - 1) * 4 + S] + g[(R - 1) * 4 + S - 1]);
+            df[((size_t)(r * 3 + s) * Cout + co) * Cinp + ci] += v;
+        }
+}
+
 }  // namespace
 
 extern "C" {
@@ -300,6 +376,16 @@ int b3d_bank_backward(const void* layers, const void* items_dot, int n_dot, cons
         B3D_LAUNCH_OK();
     }
     bank_bwd_emit_kernel<<<n_emit, NT, 0, st>>>(L, static_cast<const Item*>(items_emit), out, df, dw);
+    B3D_LAUNCH_OK();
+    return B3D_OK;
+}
+
+// dk [16][Cin][Cout] (the up-convolution's weight gradient) -> ACCUMULATED into df [9][Cout][Cinp] (the layer's F-layout
+// gradient sink)
+int b3d_bank_up2_grad(const float* dk, float* df, int Cout, int Cin, int Cinp, void* stream) {
+    B3D_REQUIRE(dk && df && Cout > 0 && Cin > 0 && Cinp >= Cin, B3D_EINVAL, "b3d_bank_up2_grad: bad arguments");
+    const long long total = (long long)Cin * Cout;
+    bank_up2_grad_kernel<<<(unsigned)((total + NT - 1) / NT), NT, 0, (cudaStream_t)stream>>>(dk, df, Cout, Cin, Cinp);
     B3D_LAUNCH_OK();
     return B3D_OK;
 }

@@ -679,7 +679,9 @@ int b3d_conv2d_tf32(const float* x, const float* wt, const float* bias, float* o
         B3D_REQUIRE(fold_kh <= 8 && Cin == 32 * ((8 * fold_kh + 31) / 32) && sy == 1 && sx == 1 && !w_cin_major && !wtap && Wout % BM == 0,
                     B3D_EINVAL, "b3d_conv2d_tf32: on-the-fly fold needs 8 input channels, stride 1 and Wout %% 128 == 0 (Wout=%d)", Wout);
     }
-    B3D_REQUIRE(!stats || mask || (osy == 1 && osx == 1), B3D_EINVAL, "b3d_conv2d_tf32: statistics need a dense output");
+    // statistics are taken over every output pixel: a dense output, or the four parity classes of a stride-2 output
+    const bool all_classes = ncls == 4 && osy == 2 && osx == 2;
+    B3D_REQUIRE(!stats || mask || (osy == 1 && osx == 1) || all_classes, B3D_EINVAL, "b3d_conv2d_tf32: statistics need a dense output");
     static const int wide = getenv("B3D_CONV_BN256") ? atoi(getenv("B3D_CONV_BN256")) : 1;
     // 256-wide output-channel tiles halve the input-tile bytes per FLOP through the L2 -> SM fabric (the bound of the
     // per-tap formulation, profiles/r1_c_*.md) when there are >= 256 output channels and enough tiles to fill the GPU
@@ -811,7 +813,8 @@ int b3d_conv2d_wgrad_tf32(const float* dy, const float* x, float* dw, int N, int
                           void* stream) {
     B3D_REQUIRE(N > 0 && Cin > 0 && Cout > 0 && H > 0 && W > 0 && Hout > 0 && Wout > 0, B3D_EINVAL,
                 "b3d_conv2d_wgrad_tf32: bad sizes");
-    B3D_REQUIRE(kh * kw <= MAX_TAPS && (stride == 1 || stride == 2) && x_off >= 0, B3D_EINVAL, "b3d_conv2d_wgrad_tf32: bad kernel/stride");
+    // x_off < 0 reads columns left of x as zeros (the TMA fills out-of-bounds boxes): the up-convolution's weight gradient
+    B3D_REQUIRE(kh * kw <= MAX_TAPS && (stride == 1 || stride == 2) && x_off > -kw, B3D_EINVAL, "b3d_conv2d_wgrad_tf32: bad kernel/stride");
     B3D_REQUIRE(dy && x && dw, B3D_EINVAL, "b3d_conv2d_wgrad_tf32: null pointer");
     B3D_REQUIRE(Cin % 32 == 0 && Cout % 32 == 0, B3D_EINVAL,
                 "b3d_conv2d_wgrad_tf32: Cin=%d and Cout=%d must be multiples of 32 (pad the channels with zeros)", Cin, Cout);

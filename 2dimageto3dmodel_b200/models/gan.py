@@ -20,7 +20,7 @@ import torch.nn.functional as F
 from b3d import B3DError
 from b3d.bank import WeightBank
 from b3d.conv import conv2d as _tc_conv2d
-from b3d.conv import ActLink, conv2d_banked
+from b3d.conv import ActLink, conv2d_banked, upconv_banked
 from b3d.ew import CIRCULAR, REPLICATE, CBNBatch, cbn_act_pad, pad_x, stem_input
 from rendering.utils import adjust_poles, symmetrize_texture
 
@@ -340,16 +340,23 @@ class ResBlockUp(nn.Module):
         from torch.nn.modules.batchnorm import _BatchNorm
         return isinstance(self.norm1.norm, _BatchNorm) and isinstance(self.norm2.norm, _BatchNorm)
 
-    def forward_fused(self, xp, z, up, pad_next, post_leaky=False, W=None, prefix="", cb=None):
+    def forward_fused(self, xp, z, up, pad_next, post_leaky=False, W=None, prefix="", cb=None, half_in=False):
         """Same block on an input that is ALREADY replicate-padded by 1 (xp = pad(x, 1)); returns the padded input of the
         consumer: pad(up(out), pad_next) with out = [LeakyReLU](h + skip).  Every conv output goes through exactly one fused
-        elementwise kernel (b3d.ew.cbn_act_pad) instead of BN, affine, LeakyReLU, add, upsample and pad kernels."""
+        elementwise kernel (b3d.ew.cbn_act_pad) instead of BN, affine, LeakyReLU, add, upsample and pad kernels.
+        half_in (banked only): xp = pad(x', 1) with x = up2(x') — conv1 runs as an up-convolution on x' and the shortcut /
+        identity skip at x''s resolution, read at (y/2, x/2) by the fused kernel (both commute with nearest upsampling)."""
         s1 = s2 = None
+        if half_in and W is None:
+            raise B3DError("ResBlockUp: a half-resolution input needs the weight bank's up-convolution taps")
         if W is not None:
             # the conv epilogues accumulate the batch-norm statistics of their output (no separate pass over y)
             if cb is not None and not getattr(self, 'disable_epilogue_stats', False):
                 s1, s2 = cb.stats_slot(self.norm1), cb.stats_slot(self.norm2)
-            c1 = lambda t: conv2d_banked(t, W[prefix + ".conv1"], pad_y=1, stats=s1)
+            if half_in:
+                c1 = lambda t: upconv_banked(t, W[prefix + ".conv1"], stats=s1)
+            else:
+                c1 = lambda t: conv2d_banked(t, W[prefix + ".conv1"], pad_y=1, stats=s1)
             c2 = lambda t: conv2d_banked(t, W[prefix + ".conv2"], pad_y=1, stats=s2)
             sc = lambda t: conv2d_banked(t, W[prefix + ".shortcut"], x_crop=1)
         else:
@@ -362,7 +369,7 @@ class ResBlockUp(nn.Module):
         else:
             skip, off = xp, 1                                        # identity: read the interior of the padded input
         return cbn_act_pad(y2, self.norm2, z, skip_nchw=skip, skip_off=off, up=up, pad=pad_next, post_leaky=post_leaky, cb=cb,
-                           sums=s2)
+                           sums=s2, skip_half=half_in)
 
 
 class Generator(nn.Module):
@@ -459,23 +466,26 @@ class Generator(nn.Module):
             return None
         bank = self.__dict__.get('_bank')
         if bank is None:
-            convs = {}
+            convs, up2 = {}, []
             for bn in ('blk1', 'blk2', 'blk3a', 'blk3b', 'blk3c', 'blk4', 'blk5', 'blk6', 'blk3_mesh'):
                 blk = getattr(self, bn, None)
                 if blk is None:
                     continue
                 convs[bn + ".conv1"], convs[bn + ".conv2"] = blk.conv1, blk.conv2
+                if bn != 'blk1':                                  # every block after the first reads an upsampled input
+                    up2.append(bn + ".conv1")
                 if isinstance(blk.shortcut, nn.Module):
                     convs[bn + ".shortcut"] = blk.shortcut
             convs["conv_final"] = self.conv_final
             if self.mesh_head:
                 convs["conv_mesh"] = self.conv_mesh
-            bank = self.__dict__['_bank'] = WeightBank(convs)
+            bank = self.__dict__['_bank'] = WeightBank(convs, up2=up2)
         return bank.forward(self.training)
 
     def _forward_fused(self, x, z, return_attention):
         """The same network with the inter-convolution glue fused (replicate-padded tensors flow between the blocks) and the
-        weights of all convolutions prepared by one WeightBank pass."""
+        weights of all convolutions prepared by one WeightBank pass.  With the bank, the blocks hand over their output BEFORE
+        the x2 upsample and every later block runs its 3x3 conv1 as an up-convolution (b3d.conv.upconv_banked)."""
         W = self._weights()
         names = [n for n in ('blk1', 'blk2', 'blk3a', 'blk3b', 'blk3c', 'blk4', 'blk5', 'blk6') if hasattr(self, n)]
         if self.mesh_head:
@@ -484,20 +494,22 @@ class Generator(nn.Module):
         cb = CBNBatch([m for n in names for m in (getattr(self, n).norm1, getattr(self, n).norm2)], z)
         blk = lambda name, inp, **kw: getattr(self, name).forward_fused(inp, z, W=W, prefix=name, cb=cb, **kw)
         head = (lambda conv, name, inp: conv(inp)) if W is None else (lambda conv, name, inp: conv2d_banked(inp, W[name], pad_y=2))
+        half = W is not None                                          # up2 happens inside the next block's conv1
+        up = 1 if half else 2
         p = pad_x(x, 1, REPLICATE)
-        p = blk('blk1', p, up=2, pad_next=1)
-        p = blk('blk2', p, up=2, pad_next=1)                          # blk2 -> up: shared by the texture and mesh branches
+        p = blk('blk1', p, up=up, pad_next=1)
+        p = blk('blk2', p, up=up, pad_next=1, half_in=half)          # blk2 -> up: shared by the texture and mesh branches
         t = p
         for name in ('blk3a', 'blk3b', 'blk3c'):
             if hasattr(self, name):
-                t = blk(name, t, up=2, pad_next=1)
-        t = blk('blk4', t, up=2, pad_next=1)
-        t = blk('blk5', t, up=2, pad_next=1)
-        t = blk('blk6', t, up=1, pad_next=2, post_leaky=True)
+                t = blk(name, t, up=up, pad_next=1, half_in=half)
+        t = blk('blk4', t, up=up, pad_next=1, half_in=half)
+        t = blk('blk5', t, up=up, pad_next=1, half_in=half)
+        t = blk('blk6', t, up=1, pad_next=2, post_leaky=True, half_in=half)
         x_tex = symmetrize_texture(torch.tanh(head(self.conv_final, "conv_final", t)))
         x_mesh = None
         if self.mesh_head:
-            m = blk('blk3_mesh', p, up=1, pad_next=2, post_leaky=True)
+            m = blk('blk3_mesh', p, up=1, pad_next=2, post_leaky=True, half_in=half)
             x_mesh = symmetrize_texture(adjust_poles(head(self.conv_mesh, "conv_mesh", m)))
         return (x_tex, x_mesh, None) if return_attention else (x_tex, x_mesh)
 

@@ -265,7 +265,8 @@ B3D_API int b3d_conv2d_tf32(const float* x, const float* wt, const float* bias, 
  * input-gradient parity classes address their tap subsets of the full weight array without a gathered copy.
  * stats (nullable): [2][Cout] fp64, ACCUMULATED into by the epilogue: per-channel sum and sum of squares of the output
  * before bias / activation — the BatchNorm statistics of the generator's layers without a second pass over the tensor
- * (models/gan.py:264-286; the caller zeroes the buffer; dense outputs only).
+ * (models/gan.py:264-286; the caller zeroes the buffer; dense outputs only, or nclass = 4 parity classes of a stride-2
+ * output, which together cover it).
  * fold_kh > 0: thin 8-channel stems (models/gan.py:163-166, 5x5 on 8 channels): x is the RAW input [N,H,W,8]; the kh vertical
  * taps are folded into the K dimension ON THE FLY by the TMA boxes (four image rows x 8 channels = one 32-channel K slice, rows
  * outside the image = the zero padding fold_pad) — Cin is the folded channel count (32 * ceil(8 kh / 32)), the taps are the kw
@@ -282,7 +283,8 @@ B3D_API int b3d_conv2d_flat_tf32(const float* x, const float* wt, const float* b
 /* Weight gradient of the same convolution (split-K tcgen05 GEMM over the output pixels, M/N-major operands
  * straight from the NHWC tensors):
  *   dw[co, ci, r, s] += sum_{n,y,x} dy[n, y, x, co] * x[n, stride*y + r - pad_y, stride*x + s + x_off, ci]
- * dy [N,Hout,Wout,Cout], x [N,H,W,Cin] (x already padded along x; Cin, Cout multiples of 4),
+ * dy [N,Hout,Wout,Cout], x [N,H,W,Cin] (x already padded along x; Cin, Cout multiples of 4; x_off > -kw: columns left
+ * of x read as zero),
  * dw [Cout,Cin,kh,kw] is ACCUMULATED into (caller zeroes it).                                          */
 B3D_API int b3d_conv2d_wgrad_tf32(const float* dy, const float* x, float* dw, int N, int H, int W, int Cin,
                                   int Hout, int Wout, int Cout, int kh, int kw, int pad_y, int stride,
@@ -341,6 +343,11 @@ B3D_API int b3d_bank_forward(const void* layers, const void* items_wtu, int n_wt
                              int training, void* stream);
 B3D_API int b3d_bank_backward(const void* layers, const void* items_dot, int n_dot, const void* items_emit, int n_emit,
                               float* out, const float* df, float* dw, void* stream);
+/* up2 layers (BankLayer.up2: a 3x3 convolution run on the input of its x2 nearest upsample as four 2x2 parity-class
+ * convolutions, class taps UF / UD written by b3d_bank_forward): the adjoint of the 3x3 -> class-tap map.  dk [4x4][Cin][Cout]
+ * is the up-convolution's weight gradient as b3d_conv2d_wgrad_tf32 (tap-major) leaves it; it is ACCUMULATED into df
+ * [9][Cout][Cinp], the layer's F-layout gradient sink. */
+B3D_API int b3d_bank_up2_grad(const float* dk, float* df, int Cout, int Cin, int Cinp, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * One-pass NHWC helpers between the GAN's convolutions.
@@ -390,18 +397,21 @@ B3D_API int b3d_bn_stats(const float* y, long long rows, int C, float eps, float
  *   out[n, yo, xo, :] = post( leaky(y[n,ys,xs,:] * scale[n,:] + shift[n,:]) + skip[n,ys,xs,:] ),
  *   (ys, xs) = (yo / up, clamp(xo - pad, 0, up*W-1) / up);  out [N, up*H, up*W + 2*pad, C];  scale = inv_std*(1+gamma),
  *   shift = beta - mean*scale ([N,C]); skip (nullable) is read at row pitch skip_pitch, pixel offset skip_off.
- * bwd1: gout -> ga = d/d(pre-activation) [N,H,W,C], gskip (nullable), S1[n,c] = sum ga, S2[n,c] = sum ga*xhat: rows of
+ *   skip_half = 1 (even H, W): the skip is at half resolution [N,H/2,..] and read at (ys/2, xs/2) — the residual of a block
+ *   whose input arrives before the x2 upsample (nearest upsampling commutes with the identity and the 1x1 shortcut).
+ * bwd1: gout -> ga = d/d(pre-activation) [N,H,W,C], gskip (nullable; skip_half: the 2x2 sums, at half resolution),
+ *       S1[n,c] = sum ga, S2[n,c] = sum ga*xhat: rows of
  *       pitch s_pitch floats (>= C; slices of the batched d(gamma, beta) buffer), zeroed by the call
  * bwd2 (in place on ga): dy = inv_std * (ga * gamma_t - m1 - xhat * m2), (m1, m2) [C] = inv_m * (sums of d xhat, d xhat * xhat)
  * b3d_cbn_prepare / b3d_cbn_bwd_reduce / b3d_bn_sums: the per-layer scalar math around these passes, one launch each
  *       (statistics -> mean / inv_std / running buffers / scale / shift; coupling-term reduction; fp64 channel sums).       */
 B3D_API int b3d_cbn_act_fwd(const float* y, const float* scale, const float* shift, const float* skip, int skip_pitch,
                             int skip_off, float* out, int N, int H, int W, int C, int up, int pad, float slope,
-                            int post_leaky, void* stream);
+                            int post_leaky, int skip_half, void* stream);
 B3D_API int b3d_cbn_act_bwd1(const float* gout, const float* y, const float* scale, const float* shift, const float* skip,
                              int skip_pitch, int skip_off, const float* mean, const float* invstd, float* ga, float* gskip,
                              int gskip_pitch, int gskip_off, float* S1, float* S2, int s_pitch, int N, int H, int W, int C,
-                             int up, int pad, float slope, int post_leaky, void* stream);
+                             int up, int pad, float slope, int post_leaky, int skip_half, void* stream);
 B3D_API int b3d_cbn_act_bwd2(float* ga, const float* y, const float* gamma_t, const float* mean, const float* invstd,
                              const float* m1, const float* m2, float inv_m, int N, int H, int W, int C, void* stream);
 B3D_API int b3d_bn_sums(const float* y, long long rows, int C, double* sums, void* stream);
